@@ -6,7 +6,7 @@ utterance, bf16, greedy (top_k=1), synthetic seeded weights at the assumed S2-Pr
 (SURVEY.md §8) — one "step" = the whole batch: prefill + 255 decode frames (+ codec decode to waveform
 once the codec stage is present in this build; `config.stages` says which stages were timed).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line.  `value` = audio-seconds generated per second (whole job, all GPUs) with the prompts
 resident in HBM; `e2e` = the same through the public API (`generate_batch`) from pinned host memory,
@@ -17,6 +17,9 @@ cores on a bounded sample.
 
 Under torchrun (N > 1) every rank runs a full replica on its own shard of utterances (32 per GPU, weak
 scaling, no collective on the data path); times are device-side, max over ranks.
+
+`--dump-outputs DIR` (batch32, one GPU) also writes what the last timed step computed as DIR/<name>.npy (see
+dump_outputs). Prompts and weights are seeded, the same on every run, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -141,6 +144,29 @@ def cpu_reference(steps: int, warmup: int):
     from oracle import cpu_baseline
 
     return cpu_baseline.measure(steps, warmup)
+
+
+DUMP_WAV_SAMPLES = 1 << 21  # 8 MiB of float32 (+ 16 MiB of float64 indices): the whole batch's waveform is 64 MiB
+
+
+def dump_outputs(out_dir: Path, codes: torch.Tensor, wav: torch.Tensor | None) -> None:
+    """What a caller of the timed path receives: `codes.npy` = the generated frames [B, C+1, NF] in float32 (row 0 the
+    semantic token ids, rows 1.. the codebook indices; every value is exact in float32) and the float32 waveform
+    [B, 1, NF*2048]: whole as `waveform.npy` when it has at most DUMP_WAV_SAMPLES samples, else a fixed seeded sample of
+    them as `waveform_sample.npy` with their flat indices (float64) in `waveform_sample_index.npy`."""
+    import numpy as np
+
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "codes.npy", codes.cpu().numpy().astype(np.float32))
+    if wav is None:
+        return
+    flat = wav.float().flatten().cpu().numpy()
+    if flat.size <= DUMP_WAV_SAMPLES:
+        np.save(out_dir / "waveform.npy", flat.reshape(tuple(wav.shape)))
+        return
+    idx = np.sort(np.random.default_rng(0).choice(flat.size, DUMP_WAV_SAMPLES, replace=False))
+    np.save(out_dir / "waveform_sample.npy", flat[idx])
+    np.save(out_dir / "waveform_sample_index.npy", idx.astype(np.float64))
 
 
 def _timed_events(fn, steps, warmup=1):
@@ -503,11 +529,18 @@ def main():
     ap.add_argument("--workload", default="batch32", choices=["batch32", "voice-clone", "serve", "single", "roundtrip", "stream"],
                     help="batch32 = BASELINE configs[2] (the headline); voice-clone = configs[4]: 10 s reference "
                          "audio -> codec encode -> ~350-position prefill -> 512 frames -> waveform, batch 8")
+    ap.add_argument("--dump-outputs", type=Path, metavar="DIR",
+                    help="write the codes and waveform of the last timed step to DIR/<name>.npy (batch32, one GPU)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.workload != "batch32" or args.impl != "b200" or world > 1
+                                          or args.profile_only):
+        ap.error("--dump-outputs covers the batch32 workload of the b200 implementation on one GPU")
     workload = (f"batch-{args.batch} text->codec->wav, {T_PROMPT}-token prompts, {args.frames} codec frames/utt, "
                 "S2-Pro 4B Dual-AR + 391M DAC codec geometry")
 
@@ -601,12 +634,14 @@ def main():
         codes = eng.buffer("out_tokens")[:B, 1:, :NF].contiguous()
         return dac.from_indices(codes)
 
+    last_wav = [None]  # waveform of the latest step_resident (--dump-outputs)
+
     def step_resident():
         eng.reset()
         eng.prefill(prompts_dev, list(range(B)), sp, do_sample=True)
         eng.decode(B, NF - 1, sp, use_graph=True)
         if not args.no_codec:
-            codec_stage()
+            last_wav[0] = codec_stage()
 
     def barrier():
         torch.cuda.synchronize()
@@ -642,6 +677,8 @@ def main():
     ms = timed(step_resident, args.steps)
     launches = _lib.launch_count() - launches0
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs is not None:  # before anything else reuses the engine's buffers
+        dump_outputs(args.dump_outputs, eng.buffer("out_tokens")[:B, :, :NF], last_wav[0])
     ms_per_step = ms / args.steps
     audio_s = B * world * NF * FRAME / SR
     value = audio_s / (ms_per_step / 1e3)

@@ -111,7 +111,8 @@ class TTSInferenceEngine(ReferenceLoader, VQManager):
             return InferenceResult(code="segment", audio=(rate, wav), error=None)
 
         # a CUDA stream of our own: the LM worker thread keeps its stream busy with decode frames meanwhile
-        side = torch.cuda.Stream(device=self.decoder_model.device) if torch.cuda.is_available() else None
+        dev = torch.device(self.decoder_model.device)
+        side = torch.cuda.Stream(device=dev) if dev.type == "cuda" else None
         while True:
             wrapped: WrappedGenerateResponse = responses.get()
             if wrapped.status == "error":

@@ -1,7 +1,9 @@
 """Host-side protocol of the drop-in boundary (no GPU): the LM worker queue
 (launch_thread_safe_queue, inference.py:736-799) and TTSInferenceEngine.inference
 (inference_engine/__init__.py:40-142) with the device work replaced by stand-ins."""
+import json
 import queue
+from pathlib import Path
 
 import numpy as np
 import pytest
@@ -515,28 +517,67 @@ class _ByteTokenizer:
         return ids
 
 
-def test_generate_long_plan_builds_growing_prompts_with_the_reference_frontend():
-    """The REAL body of the generate_long plan (inference.py:523-733) on CPU: the reference's own prompt builder
-    (fish_speech.content_sequence / conversation from /root/reference) with a byte-level tokenizer, a driver that answers
-    every `generate` with a made-up continuation. Checks what the CUDA side relies on: every chunk's prompt EXTENDS the
-    previous chunk's prompt (prefix K/V reuse, SURVEY §8(f).2), the reference clip enters as semantic rows, each chunk
-    yields y[1:, T:-1] (the last frame is dropped, :708) and the stream ends with "next"."""
-    import sys
-    from pathlib import Path
+FRONTEND_GOLD = Path(__file__).parent / "golden" / "generate_long_frontend.npz"
 
-    ref = Path("/root/reference")
-    if not (ref / "fish_speech" / "conversation.py").exists():
-        pytest.skip("the reference checkout (CPU-side prompt builder) is not available")
-    if str(ref) not in sys.path:
-        sys.path.insert(0, str(ref))
+
+def _frontend_value(v):
+    """JSON form of an argument the generate_long plan passes to the prompt builder (nested parts and tensors included)."""
+    if isinstance(v, torch.Tensor):
+        return {"dtype": str(v.dtype), "shape": list(v.shape), "values": v.flatten().tolist()}
+    if isinstance(v, (list, tuple)):
+        return [_frontend_value(x) for x in v]
+    if hasattr(v, "frontend_call"):
+        kind, kw = v.frontend_call
+        return {"kind": kind, **{k: _frontend_value(x) for k, x in kw.items()}}
+    return v
+
+
+def frontend_conversation_json(messages) -> str:
+    """Every Message of a conversation as the plan constructed it (constructor, keyword arguments, parts)."""
+    return json.dumps([_frontend_value(m) for m in messages], sort_keys=True)
+
+
+def _recorded_frontend(gold):
+    """Stand-in for the reference's prompt builder (fish_speech.conversation / content_sequence) that replays a recorded
+    run of the real one (oracle/make_golden_frontend.py): the k-th encode_for_inference must be asked to encode exactly
+    the conversation the reference encoded k-th, and returns the reference's prompt for it."""
+    calls = iter(range(len(gold["conversations"])))
+
+    class Call:
+        def __init__(self, kind, **kw):
+            self.frontend_call = (kind, kw)
+
+    class Conversation:
+        def __init__(self):
+            self.messages = []
+
+        def append(self, message):
+            self.messages.append(message)
+
+        def encode_for_inference(self, tokenizer, num_codebooks):
+            k = next(calls, None)
+            assert k is not None, "the plan encodes more prompts than the recorded reference run"
+            assert num_codebooks == int(gold["num_codebooks"])
+            assert frontend_conversation_json(self.messages) == str(gold["conversations"][k]), \
+                f"prompt {k}: the plan built a different conversation than the recorded reference run"
+            return torch.from_numpy(gold[f"encoded_{k}"]), None, None
+
+    def part(kind):
+        return lambda **kw: Call(kind, **kw)
+
+    return part("TextPart"), part("VQPart"), Conversation, part("Message")
+
+
+def drive_generate_long_plan(tok):
+    """The REAL body of the generate_long plan (inference.py:523-733) with a byte-level tokenizer and a driver that
+    answers every `generate` with a made-up continuation. Returns (prompts, responses, reference clip codes)."""
 
     class Model:
         class config:
             max_seq_len, num_codebooks = 8192, 10
 
-        tokenizer = _ByteTokenizer()
+        tokenizer = tok
 
-    tok = Model.tokenizer
     ref_codes = torch.arange(10 * 6).view(10, 6) % 1024
     text = "<|speaker:0|>" + "first sentence of the request. " * 3 + "<|speaker:1|>" + "and a reply that is long enough. " * 3
     plan = inf._generate_long_plan(model=Model, device="cpu", text=text, chunk_length=100, max_new_tokens=64,
@@ -563,6 +604,21 @@ def test_generate_long_plan_builds_growing_prompts_with_the_reference_frontend()
         gen[1:] = (torch.arange(10).view(10, 1) + fake_frames) % 1024
         gen[0, -1] = tok.get_token_id("<|im_end|>")
         reply = torch.cat([p, gen], dim=1)
+    return prompts, responses, ref_codes
+
+
+def test_generate_long_plan_builds_growing_prompts_with_the_reference_frontend(monkeypatch):
+    """The generate_long plan against a recorded run of the reference's own prompt builder (fish_speech.content_sequence /
+    conversation, tests/golden/generate_long_frontend.npz): the plan must hand the builder the same conversations, chunk
+    by chunk. Checks on the reference's prompts what the CUDA side relies on: every chunk's prompt EXTENDS the previous
+    chunk's prompt (prefix K/V reuse, SURVEY §8(f).2), the reference clip enters as semantic rows, each chunk yields
+    y[1:, T:-1] (the last frame is dropped, :708) and the stream ends with "next"."""
+    gold = np.load(FRONTEND_GOLD)
+    monkeypatch.setattr(inf, "_reference_frontend", lambda: _recorded_frontend(gold))
+    tok = _ByteTokenizer()
+    tok.special = json.loads(str(gold["tokenizer_special"]))
+    prompts, responses, ref_codes = drive_generate_long_plan(tok)
+    assert len(prompts) == len(gold["conversations"])
     assert len(prompts) >= 2, "the text must split into several chunks"
     # the reference clip: semantic ids on row 0, its codes on rows 1..10
     first = prompts[0]
