@@ -105,6 +105,11 @@ def lib() -> C.CDLL:
     L.fsb_window_attn.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
     L.fsb_swiglu_f32.argtypes = [vp, i32, i32, vp, vp]
     L.fsb_op_gemm.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, vp]
+    L.fsb_op_step_gemm.argtypes = [vp, i32, i32, vp, i32, i32, vp, i32, vp, C.c_float, i32, i32, vp, C.c_size_t,
+                                   vp, i32p, i32p, i32p, vp]
+    L.fsb_op_step_finalize.argtypes = [i32, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, i32, vp]
+    L.fsb_op_attn_decode.argtypes = [vp, vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32,
+                                     i32, i32, i32, C.c_float, vp]
     _lib = L
     return L
 

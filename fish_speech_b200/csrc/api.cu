@@ -99,4 +99,99 @@ int fsb_op_gemm(const void* d_a, const void* d_b, float* d_out, int m, int n, in
     return 0;
 }
 
+int fsb_op_step_gemm(const void* d_w, int n_out, int K, const void* d_x, int rows, int norm_on_load,
+                     const float* d_x_ssq, int x_nt, const void* d_norm_w, float eps, int num_ctas, int stages,
+                     float* d_ws, size_t ws_floats, int32_t* h_nparts, int* max_parts, int* grid, int* stages_used,
+                     void* stream) {
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    FSB_CHECK(rows >= 1 && rows <= kStepRows, "step GEMM hook: rows=%d", rows);
+    FSB_CHECK(!norm_on_load || (x_nt >= 1 && x_nt <= kSsqStride && d_x_ssq && d_norm_w), "step GEMM hook: norm inputs");
+    StepGemmPlan plan;
+    FSB_TRY(step_plan_init(&plan, reinterpret_cast<const __nv_bfloat16*>(d_w), n_out, K,
+                           reinterpret_cast<const __nv_bfloat16*>(d_x), norm_on_load != 0, num_ctas, stages, d_ws,
+                           ws_floats));
+    plan.p.rows = rows;
+    if (norm_on_load) {
+        plan.p.x_ssq = d_x_ssq;
+        plan.p.norm_w = reinterpret_cast<const __nv_bfloat16*>(d_norm_w);
+        plan.p.x_nt = x_nt;
+        plan.p.eps = eps;
+    }
+    int rc = step_gemm_launch(plan, st);
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (rc == 0 && e == cudaSuccess)
+        e = cudaMemcpy(h_nparts, plan.nparts_dev, plan.p.tiles * sizeof(int32_t), cudaMemcpyDeviceToHost);
+    *max_parts = plan.max_parts;
+    *grid = static_cast<int>(plan.grid.x);
+    *stages_used = plan.p.stages;
+    step_plan_free(&plan);
+    if (rc != 0) return rc;
+    FSB_CUDA(e);
+    return 0;
+}
+
+// The consumer-side plan of a partial set as the hooks below receive it (slot-major layout of StepPartials).
+static StepPartials hook_partials(const float* d_ws, const int32_t* d_nparts, int tiles, int n_out, int max_parts) {
+    StepPartials P;
+    P.ws = d_ws;
+    P.nparts = d_nparts;
+    P.tiles = tiles;
+    P.n_out = n_out;
+    P.max_parts = max_parts;
+    return P;
+}
+
+int fsb_op_step_finalize(int pro, const float* d_ws, const int32_t* d_nparts, int tiles, int n_out, int max_parts,
+                         int rows, int rb, const void* d_bias, const void* d_resid, void* d_x_out, float* d_ssq_out,
+                         void* d_h, int I, void* stream) {
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    FSB_CHECK(pro == PRO_RESID || pro == PRO_SWIGLU, "finalize hook: pro=%d", pro);
+    FSB_CHECK(rows >= 1 && rows <= kStepRows && max_parts >= 1 && tiles == cdiv(n_out, 128), "finalize hook: shape");
+    FSB_CHECK(pro != PRO_RESID || (d_x_out && d_ssq_out && tiles <= kSsqStride), "finalize hook: residual outputs");
+    FSB_CHECK(pro != PRO_SWIGLU || (d_h && I >= 1 && I <= tiles * 64), "finalize hook: SwiGLU output");
+    StepGemmPlan consumer;
+    memset(&consumer, 0, sizeof(consumer));
+    consumer.pro = pro;
+    consumer.p.prev = hook_partials(d_ws, d_nparts, tiles, n_out, max_parts);
+    consumer.p.rows = rows;
+    consumer.p.bias = reinterpret_cast<const __nv_bfloat16*>(d_bias);
+    consumer.p.resid = reinterpret_cast<const __nv_bfloat16*>(d_resid);
+    consumer.p.x_out = reinterpret_cast<__nv_bfloat16*>(d_x_out);
+    consumer.p.ssq_out = d_ssq_out;
+    consumer.p.h = reinterpret_cast<__nv_bfloat16*>(d_h);
+    consumer.p.I = I;
+    FSB_TRY(step_finalize_launch(consumer, st, rb));
+    FSB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+int fsb_op_attn_decode(const float* d_ws, const int32_t* d_nparts, int tiles, int max_parts, const void* d_bias,
+                       const void* d_q_norm, const void* d_k_norm, const void* d_freqs, void* d_kcache, void* d_vcache,
+                       const int32_t* d_row_seq, const int32_t* d_row_pos, void* d_out, int rows, int H, int Hkv,
+                       int Dh, int S, int lcap, int bf16_math, int kv_only, float eps, void* stream) {
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    const int n_out = (H + 2 * Hkv) * Dh;
+    FSB_CHECK(rows >= 1 && rows <= kStepRows && max_parts >= 1 && tiles == cdiv(n_out, 128), "attention hook: shape");
+    FSB_TRY(attn_init());
+    AttnDecodeArgs a{};
+    a.qkv = hook_partials(d_ws, d_nparts, tiles, n_out, max_parts);
+    a.bias = reinterpret_cast<const __nv_bfloat16*>(d_bias);
+    a.q_norm = reinterpret_cast<const __nv_bfloat16*>(d_q_norm);
+    a.k_norm = reinterpret_cast<const __nv_bfloat16*>(d_k_norm);
+    a.freqs = reinterpret_cast<const __nv_bfloat16*>(d_freqs);
+    a.kcache = reinterpret_cast<__nv_bfloat16*>(d_kcache);
+    a.vcache = reinterpret_cast<__nv_bfloat16*>(d_vcache);
+    a.row_seq = d_row_seq;
+    a.row_pos = d_row_pos;
+    a.out = reinterpret_cast<__nv_bfloat16*>(d_out);
+    a.rows = rows; a.H = H; a.Hkv = Hkv; a.Dh = Dh; a.S = S;
+    a.lcap = lcap;
+    a.bf16_math = bf16_math;
+    a.kv_only = kv_only;
+    a.eps = eps;
+    FSB_TRY(launch_attn_decode(a, st));
+    FSB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
 }  // extern "C"

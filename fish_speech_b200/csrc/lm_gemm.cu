@@ -434,6 +434,8 @@ int step_plan_init(StepGemmPlan* plan, const __nv_bfloat16* w, int n_out, int K,
     memset(plan, 0, sizeof(*plan));
     FSB_CHECK(K % 8 == 0, "step GEMM: K=%d must be a multiple of 8", K);
     FSB_CHECK(act != nullptr, "step GEMM: operand X missing");
+    FSB_CHECK(!norm_on_load || cdiv(K, 128) <= kSsqStride, "step GEMM: normalise-on-load needs K <= %d (K=%d)",
+              kSsqStride * 128, K);
     const int norm = norm_on_load ? 1 : 0;
     const void* kernel = kernel_of(norm);
     FSB_TRY(step_gemm_init());
@@ -542,7 +544,7 @@ void step_plan_free(StepGemmPlan* plan) {
     plan->nparts_dev = nullptr;
 }
 
-int step_finalize_launch(const StepGemmPlan& consumer, cudaStream_t st) {
+int step_finalize_launch(const StepGemmPlan& consumer, cudaStream_t st, int rb) {
     // `consumer`'s finalize fields (prev, bias / resid / x_out / ssq_out or h / I, rows) describe the work; one unit per CTA
     const int pro = consumer.pro;
     if (pro == PRO_NONE) return 0;
@@ -550,7 +552,7 @@ int step_finalize_launch(const StepGemmPlan& consumer, cudaStream_t st) {
     // one load round per unit (<= 4 / <= 16 partials), every unit on its own CTA
     static const int rb_swiglu = [] { const char* e = getenv("FSB_SWIGLU_RB"); return e ? atoi(e) : 8; }();
     static const int rb_resid = [] { const char* e = getenv("FSB_RESID_RB"); return e ? atoi(e) : 2; }();
-    const int rb = pro == PRO_SWIGLU ? rb_swiglu : rb_resid;
+    if (rb <= 0) rb = pro == PRO_SWIGLU ? rb_swiglu : rb_resid;
     FSB_CHECK(rb >= 1 && rb <= 32 && (rb & (rb - 1)) == 0, "finalize: row block %d is not a power of two <= 32", rb);
     p.prev_rb = rb;
     const int units = p.prev.tiles * cdiv(p.rows, rb);

@@ -150,8 +150,9 @@ StepPartials step_plan_partials(const StepGemmPlan& plan);
 void step_plan_set_prev(StepGemmPlan* plan, int pro, const StepGemmPlan& prev);
 void step_plan_free(StepGemmPlan* plan);
 int step_gemm_launch(const StepGemmPlan& plan, cudaStream_t stream);
-// finish the GEMM that produces `consumer`'s operand (no-op when consumer.pro == PRO_NONE); launch it before the consumer
-int step_finalize_launch(const StepGemmPlan& consumer, cudaStream_t stream);
+// finish the GEMM that produces `consumer`'s operand (no-op when consumer.pro == PRO_NONE); launch it before the consumer.
+// rb: batch rows per finalize unit (power of two <= 32); 0 = FSB_SWIGLU_RB / FSB_RESID_RB or the default (8 / 2)
+int step_finalize_launch(const StepGemmPlan& consumer, cudaStream_t stream, int rb = 0);
 int step_gemm_init();  // kernel attributes (idempotent)
 
 // Row index of the fused w1|w3 weight for SwiGLU: h feature f -> row of w1[f]; w3[f] sits 16 rows further.

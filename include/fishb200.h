@@ -253,6 +253,31 @@ int fsb_swiglu_f32(const float* d_y, int rows, int I, void* d_h, void* stream);
 int fsb_op_gemm(const void* d_a, const void* d_b, float* d_out, int m, int n, int k, int bn,
                 int streamk_ctas, void* stream);
 
+/* The decode step's kernels one at a time, through the host code the decode frame uses (csrc/lm_gemm.cu,
+ * csrc/lm_kernels.cu). Each call synchronises `stream`. A partial set is the stream-K output of one step GEMM:
+ *   value(row j, feature i) = sum over slots q < nparts[i/128], in slot order, of
+ *                             ws[((q * tiles + i/128) * 32 + j) * 128 + i%128]
+ * fsb_op_step_gemm: partials of W [n_out, K] x X [32, K]^T for batch rows [0, rows) into the caller's d_ws
+ * (ws_floats floats; slots >= nparts of a tile and rows >= rows are not written). norm_on_load != 0: X is the
+ * residual stream, normalised on load with d_x_ssq [32][32] (x_nt per-128-feature sums of squares per row),
+ * d_norm_w [K] and eps. Returns nparts [ceil(n_out/128)] in h_nparts, the slot count, the grid and the ring depth. */
+int fsb_op_step_gemm(const void* d_w, int n_out, int K, const void* d_x, int rows, int norm_on_load,
+                     const float* d_x_ssq, int x_nt, const void* d_norm_w, float eps, int num_ctas, int stages,
+                     float* d_ws, size_t ws_floats, int32_t* h_nparts, int* max_parts, int* grid, int* stages_used,
+                     void* stream);
+/* step_finalize over a partial set (d_nparts on the device) with `rb` batch rows per unit (0 = the default):
+ * pro 1 = residual add: x_out = rbf(resid + rbf(sum + bias)), ssq_out [32][32] per-tile sums of squares
+ * (d_bias, d_resid optional; d_resid may alias d_x_out); pro 2 = SwiGLU on the interleaved w1|w3 result into d_h [rows][I]. */
+int fsb_op_step_finalize(int pro, const float* d_ws, const int32_t* d_nparts, int tiles, int n_out, int max_parts,
+                         int rows, int rb, const void* d_bias, const void* d_resid, void* d_x_out, float* d_ssq_out,
+                         void* d_h, int I, void* stream);
+/* Decode attention over a qkv partial set (n_out = (H + 2*Hkv) * Dh): bias, q/k RMSNorm, RoPE, KV append at
+ * [row_seq][g][row_pos], attention into d_out [rows][H*Dh]; the fields of the decode frame's call, all exposed. */
+int fsb_op_attn_decode(const float* d_ws, const int32_t* d_nparts, int tiles, int max_parts, const void* d_bias,
+                       const void* d_q_norm, const void* d_k_norm, const void* d_freqs, void* d_kcache, void* d_vcache,
+                       const int32_t* d_row_seq, const int32_t* d_row_pos, void* d_out, int rows, int H, int Hkv,
+                       int Dh, int S, int lcap, int bf16_math, int kv_only, float eps, void* stream);
+
 /* Attention keeps one fp32 score per position and head in shared memory; contexts longer than the buffer are walked
  * in chunks, bit-identically (csrc/lm_kernels.cu attend()).  positions > 0 forces a smaller chunk; 0 = automatic. */
 int fsb_op_attn_score_chunk(int positions);

@@ -1,4 +1,7 @@
-"""tcgen05/TMA GEMM (csrc/gemm_tc.cu) against an fp32 matmul of the same bf16 operands."""
+"""tcgen05/TMA GEMM of prefill and the codec (csrc/gemm_tc.cu) against an fp32 matmul of the same bf16 operands.
+
+The stream-K cases run gemm_tc.cu's own stream-K schedule (gemm_plan_streamk), not the decode step GEMM of
+csrc/lm_gemm.cu; that one and its finalize are tested op by op in test_step_gpu.py."""
 import pytest
 import torch
 
@@ -44,9 +47,9 @@ def test_gemm_direct(m, n, k, bn):
     (128, 32, 256, 1),
     (128, 32, 256, 3),      # split one tile over 3 CTAs
     (640, 32, 2560, 148),   # many segments, ragged ranges
-    (6144, 32, 2560, 148),  # wqkv shape
-    (2560, 8, 9728, 148),   # w2 shape, small batch
-    (4097, 5, 2560, 148),   # restricted LM head
+    (6144, 32, 2560, 148),  # many tiles, about 3 segments per tile
+    (2560, 8, 9728, 148),   # long K: about 8 segments per tile, 8 columns
+    (4097, 5, 2560, 148),   # a last tile of one row, 5 columns
 ])
 def test_gemm_streamk(m, n, k, ctas):
     _run(m, n, k, 32, ctas)
