@@ -101,7 +101,6 @@ def lib() -> C.CDLL:
     L.fsb_res_unit.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.fsb_op_res_unit_trace.argtypes = [vp]
     L.fsb_op_attn_score_chunk.argtypes = [i32]
-    L.fsb_op_attn_per_row.argtypes = [i32]
     L.fsb_window_attn.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]
     L.fsb_swiglu_f32.argtypes = [vp, i32, i32, vp, vp]
     L.fsb_op_gemm.argtypes = [vp, vp, vp, i32, i32, i32, i32, i32, vp]

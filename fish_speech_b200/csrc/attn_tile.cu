@@ -1,15 +1,15 @@
 // Tiled attention on the tensor cores for MANY query rows per sequence: LM prefill (llama.py:916-934 with S > 1) and the
-// codec's window-limited transformer (modded_dac.py:380-398).  The per-row kernel (lm_kernels.cu attn_kernel) re-reads
-// the whole K/V history of a row from L2 for every row: O(L^2) bytes and CUDA-core dot products.  Here one CTA takes 64
-// consecutive rows of one query head: K/V tiles of 64 positions are staged once in shared memory (cp.async, double
-// buffered) and shared by the 64 rows, S = Q K^T and O += P V run on mma.sync m16n8k16 (bf16 in, fp32 accumulate; the
-// probabilities as a bf16 hi + lo pair), the softmax is the online (running max / running sum) form in fp32.
+// codec's window-limited transformer (modded_dac.py:380-398).  A kernel per row would re-read the whole K/V history of
+// a row from L2 for every row: O(L^2) bytes and CUDA-core dot products.  Here one CTA takes 64 consecutive rows of one
+// query head: K/V tiles of 64 positions are staged once in shared memory (cp.async, double buffered) and shared by the
+// 64 rows, S = Q K^T and O += P V run on mma.sync m16n8k16 (bf16 in, fp32 accumulate; the probabilities as a bf16
+// hi + lo pair), the softmax is the online (running max / running sum) form in fp32.
 //
-// Rows come as in the per-row kernel: arbitrary (sequence, position) per row.  A tile is split into runs of consecutive
-// positions of one sequence; each run is processed against its own K/V range with the other rows masked (a fully masked
-// K tile leaves a row's running state untouched).  K tiles are aligned to absolute multiples of 64 positions and a
-// row's result only depends on its own positions, so a prompt gives the same bits however it is cut into prefill
-// chunks or grouped into tiles (prefix reuse relies on this).
+// Each row has its own (sequence, position).  A tile is split into runs of consecutive positions of one sequence; each
+// run is processed against its own K/V range with the other rows masked (a fully masked K tile leaves a row's running
+// state untouched).  K tiles are aligned to absolute multiples of 64 positions and a row's result only depends on its
+// own positions, so a prompt gives the same bits however it is cut into prefill chunks or grouped into tiles (prefix
+// reuse relies on this).
 #include "lm_kernels.cuh"
 
 namespace fsb {
@@ -209,7 +209,7 @@ __global__ void __launch_bounds__(kAtThreads) attn_tile_kernel(AttnArgs a, float
         }
         start = end;
     }
-    // ---- O / l -> bf16; rows without a position (idle slots) read as zero, like the per-row kernel ----
+    // ---- O / l -> bf16; rows without a position (idle slots) read as zero ----
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
         const int qi = h == 0 ? qi0 : qi1;
@@ -238,13 +238,10 @@ int launch_t(const AttnArgs& a, cudaStream_t st) {
 
 }  // namespace
 
-bool attn_tile_supported(const AttnArgs& a) {
-    return a.bf16_math == 0 && (a.Dh == 64 || a.Dh == 128) && a.H % a.Hkv == 0;
-}
-
-int launch_attn_tile(const AttnArgs& a, cudaStream_t st) {
+int launch_attn(const AttnArgs& a, cudaStream_t st) {
     if (a.rows <= 0) return 0;
-    FSB_CHECK(attn_tile_supported(a), "attn_tile: unsupported geometry (head_dim %d)", a.Dh);
+    FSB_CHECK((a.Dh == 64 || a.Dh == 128) && a.Hkv > 0 && a.H % a.Hkv == 0,
+              "attention: unsupported geometry (head_dim %d, %d heads, %d KV heads)", a.Dh, a.H, a.Hkv);
     return a.Dh == 64 ? launch_t<64>(a, st) : launch_t<128>(a, st);
 }
 

@@ -508,7 +508,6 @@ int fsb_qkv_rope(const float* d_qkv, int rows, int H, int Hkv, int Dh, const voi
 int fsb_window_attn(const void* d_q, const void* d_k, const void* d_v, const int32_t* d_row_seq,
                     const int32_t* d_row_pos, int rows, int H, int Hkv, int Dh, int S, int window, void* d_out,
                     void* stream) {
-    FSB_TRY(attn_init());
     AttnArgs a{};
     a.q = reinterpret_cast<const bf16*>(d_q);
     a.kcache = reinterpret_cast<const bf16*>(d_k);
@@ -518,16 +517,11 @@ int fsb_window_attn(const void* d_q, const void* d_k, const void* d_v, const int
     a.out = reinterpret_cast<bf16*>(d_out);
     a.rows = rows; a.H = H; a.Hkv = Hkv; a.Dh = Dh; a.S = S;
     a.window = window;
-    a.bf16_math = 0;
     return launch_attn(a, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int fsb_op_attn_score_chunk(int positions) {
     attn_set_score_chunk(positions);
-    return 0;
-}
-int fsb_op_attn_per_row(int on) {
-    attn_force_per_row(on != 0);
     return 0;
 }
 

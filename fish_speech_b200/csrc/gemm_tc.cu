@@ -254,19 +254,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         }
                     }
                 }
-                // ... and the next `l2_prefetch` k-blocks go to L2: the HBM stream of this GEMM keeps
-                // running through the tail of the previous kernel and the small consumer kernel between.
-                for (int q = 0; q < p.l2_prefetch && n < item_end; ++q) {
-                    const int tap = kb / p.kb_per_tap;
-                    const int kc = (kb - tap * p.kb_per_tap) * kBlockK;
-                    tma_prefetch_l2_3d(&tmA, p.a_tapk * tap + kc, i0 + p.a_shift[tap], p.a_batched ? z : 0);
-                    if (++kb >= kb1) {
-                        if (++n < item_end) {
-                            get_item(n, i0, j0, kb0, kb1, slot);
-                            kb = kb0;
-                        }
-                    }
-                }
             }
             pdl_wait();
             for (int n = item_begin; n < item_end; ++n) {

@@ -30,7 +30,6 @@ struct GemmParams {
     unsigned long long a_hint, b_hint;         // L2 eviction policy per operand
     int stages;
     int a_static;  // operand A is constant data (weights): prefetch it before griddepcontrol.wait
-    int l2_prefetch;  // extra k-blocks of A per CTA prefetched into L2 before the wait
     // ---- work decomposition ----
     const int4* sched;     // optional items {tile_i | tile_j<<16, kb_begin, kb_end, slot}; else blockIdx
     const int* cta_items;  // [grid.x + 1] item range of each CTA (stream-K)

@@ -18,8 +18,6 @@
 //
 // Reference: fish_speech/models/text2semantic/llama.py:390-466 (slow step), :799-817 (fast step),
 // fish_speech/models/text2semantic/inference.py:96-181 (one frame), :184-238 (frame loop).
-#include <stdlib.h>
-
 #include <algorithm>
 #include <map>
 #include <string>
@@ -36,6 +34,9 @@ namespace {
 
 typedef __nv_bfloat16 bf16;
 constexpr int kDecRows = kStepRows;  // decode GEMM N tile: up to 32 sequences per step
+// step GEMM ring depth and resident CTAs per SM: measured best (profiles/r02_decode_structure.md item 7)
+constexpr int kStepStages = 4;
+constexpr int kStepCtasPerSm = 2;
 
 struct LayerW {
     const bf16 *attn_norm, *wqkv, *bqkv, *q_norm, *k_norm, *wo, *bo, *ffn_norm, *w13, *w2;
@@ -77,7 +78,7 @@ struct fsb_lm {
     bool graph_slot_control = false;
     fsb_lm_config cfg;
     int num_sms = 148;
-    int step_ctas = 0, step_stages = 4;
+    int step_ctas = 0;
     Stack slow, fast;
     const bf16 *emb = nullptr, *cb_emb = nullptr, *norm_w = nullptr, *head_w = nullptr;
     const bf16 *fast_emb = nullptr, *fast_norm_w = nullptr, *fast_out_w = nullptr;
@@ -165,9 +166,8 @@ int launch_rows_of(const GemmPlan& plan, int rows, cudaStream_t st) {
 }
 
 int launch_rows_of(const GemmPlan& plan, const GemmPlan& wide, int rows, cudaStream_t st) {
-    static const bool on = [] { const char* e = getenv("FSB_PREFILL_WIDE"); return !(e && e[0] == '0'); }();
     const long long tiles_wide = static_cast<long long>(wide.grid.x) * cdiv(rows, 256);
-    return (on && rows >= 512 && tiles_wide >= 296) ? launch_rows_of(wide, rows, st) : launch_rows_of(plan, rows, st);
+    return (rows >= 512 && tiles_wide >= 296) ? launch_rows_of(wide, rows, st) : launch_rows_of(plan, rows, st);
 }
 
 // Step GEMM over the weight `w` [n_out, K]. act != null: operand X = act, used as it is; act == null: operand X = the
@@ -176,7 +176,18 @@ int make_step_plan(fsb_lm* h, StepGemmPlan* plan, const bf16* w, int n_out, int 
                    const Stack* norm_of = nullptr) {
     const bool norm = act == nullptr;
     if (norm) act = norm_of->xres;
-    return step_plan_init(plan, w, n_out, K, act, norm, h->step_ctas, h->step_stages, h->step_ws, h->step_ws_floats);
+    return step_plan_init(plan, w, n_out, K, act, norm, h->step_ctas, kStepStages, h->step_ws, h->step_ws_floats);
+}
+
+// Finish the GEMM that produces `plan`'s operand (residual add / SwiGLU), then launch `plan` itself over `rows` batch
+// rows; under fsb_lm_trace_frame the step GEMM records its per-CTA stamps.
+int launch_step(fsb_lm* h, const StepGemmPlan& plan, int rows, cudaStream_t st) {
+    StepGemmPlan q = plan;
+    q.p.rows = rows;
+    FSB_TRY(step_finalize_launch(q, st));
+    if (h->trace_base && h->trace_next < h->trace_max && q.grid.x <= 512)
+        q.p.trace = h->trace_base + static_cast<size_t>(h->trace_next++) * 8 * 512;
+    return step_gemm_launch(q, st);
 }
 
 void bind_norm_on_load(StepGemmPlan* plan, const Stack& s, const bf16* norm_w, float eps) {
@@ -214,20 +225,11 @@ SlotCtl slot_ctl(const fsb_lm* h) {
 int run_stack_decode(fsb_lm* h, Stack& s, int rows, const int* row_seq, const int* row_pos, bool stop_after_kv,
                      cudaStream_t st, const StepGemmPlan* first_qkv = nullptr) {
     const float eps = h->cfg.norm_eps;
-    // finish the producer of the operand (residual add / SwiGLU), then the GEMM itself
-    auto launch = [&](const StepGemmPlan& plan) -> int {
-        StepGemmPlan q = plan;
-        q.p.rows = rows;
-        FSB_TRY(step_finalize_launch(q, st));
-        if (h->trace_base && h->trace_next < h->trace_max && q.grid.x <= 512)
-            q.p.trace = h->trace_base + static_cast<size_t>(h->trace_next++) * 8 * 512;
-        return step_gemm_launch(q, st);
-    };
     for (int l = 0; l < s.nl; ++l) {
         StepLayer& P = s.dec[l];
         const LayerW& w = s.w[l];
         const StepGemmPlan& qkv = (l == 0 && first_qkv) ? *first_qkv : P.qkv;
-        FSB_TRY(launch(qkv));
+        FSB_TRY(launch_step(h, qkv, rows, st));
         AttnDecodeArgs aa{};
         aa.qkv = step_plan_partials(qkv);
         aa.bias = w.bqkv;
@@ -248,9 +250,9 @@ int run_stack_decode(fsb_lm* h, Stack& s, int rows, const int* row_seq, const in
             aa.trace = h->attn_trace_base + static_cast<size_t>(h->attn_trace_next++) * 8;
         FSB_TRY(launch_attn_decode(aa, st));
         if (aa.kv_only) return 0;
-        FSB_TRY(launch(P.wo));
-        FSB_TRY(launch(P.w13));
-        FSB_TRY(launch(P.w2));
+        FSB_TRY(launch_step(h, P.wo, rows, st));
+        FSB_TRY(launch_step(h, P.w13, rows, st));
+        FSB_TRY(launch_step(h, P.w2, rows, st));
     }
     return 0;
 }
@@ -287,8 +289,6 @@ int run_stack_prefill(fsb_lm* h, Stack& s, int rows, const int* row_seq, const i
         aa.out = h->attn_p;
         aa.rows = rows; aa.H = s.H; aa.Hkv = s.Hkv; aa.Dh = s.Dh; aa.S = s.S;
         aa.window = 0;
-        aa.lcap = h->ctx_lcap;
-        aa.bf16_math = 0;
         FSB_TRY(launch_attn(aa, st));
         FSB_TRY(launch_rows_of(P.wo, rows, st));
         ResidNormArgs r1{};
@@ -326,14 +326,6 @@ int run_frame_tail(fsb_lm* h, int rows, const int* row_slot, bool use_ras, const
     const int* slots = row_slot ? row_slot : h->iota;
     Stack& s = h->slow;
     Stack& f = h->fast;
-    auto launch = [&](const StepGemmPlan& plan) -> int {
-        StepGemmPlan q = plan;
-        q.p.rows = rows;
-        FSB_TRY(step_finalize_launch(q, st));
-        if (h->trace_base && h->trace_next < h->trace_max && q.grid.x <= 512)
-            q.p.trace = h->trace_base + static_cast<size_t>(h->trace_next++) * 8 * 512;
-        return step_gemm_launch(q, st);
-    };
     auto sample_args = [&](int n, const StepGemmPlan& head) {
         SampleArgs a{};
         a.ctl = slot_ctl(h);
@@ -354,7 +346,7 @@ int run_frame_tail(fsb_lm* h, int rows, const int* row_slot, bool use_ras, const
     // ---- slow head over the selectable rows (first the last layer's FFN output is added to the residual stream,
     // unless the rows come from a prefill; the final norm is applied on load) ----
     const StepGemmPlan& head = x_is_final ? h->head_plan_direct : h->head_plan;
-    FSB_TRY(launch(head));
+    FSB_TRY(launch_step(h, head, rows, st));
     SampleArgs sa = sample_args(h->head_rows, head);
     sa.slow = 1;
     sa.n_sem = h->head_rows - 1;
@@ -379,7 +371,8 @@ int run_frame_tail(fsb_lm* h, int rows, const int* row_slot, bool use_ras, const
     if (h->has_proj) {
         hr.y = h->hid_d;
         FSB_TRY(launch_rows(hr, st));
-        FSB_TRY(launch(h->proj_plan));  // fast_project_in; the finalize in front of layer 0's qkv GEMM adds the bias
+        // fast_project_in; the finalize in front of layer 0's qkv GEMM adds the bias
+        FSB_TRY(launch_step(h, h->proj_plan, rows, st));
     } else {
         hr.y = f.xres;
         hr.ssq = f.ssq;
@@ -401,7 +394,7 @@ int run_frame_tail(fsb_lm* h, int rows, const int* row_slot, bool use_ras, const
         FSB_TRY(run_stack_decode(h, f, rows, slots, h->fpos + p * kDecRows, p == 0, st,
                                  (p == 0 && h->has_proj) ? &h->fast_qkv0_proj : nullptr));
         if (p == 0) continue;
-        FSB_TRY(launch(h->fast_out_plan));
+        FSB_TRY(launch_step(h, h->fast_out_plan, rows, st));
         SampleArgs fa = sample_args(c.codebook_size, h->fast_out_plan);
         fa.slow = 0;
         fa.draw_id = p;
@@ -481,14 +474,7 @@ int fsb_lm_create(const fsb_lm_config* cfg, const fsb_lm_weights* w, fsb_lm** ou
         delete h;
         return 1;
     }
-    {
-        // ring depth / CTAs per SM of the step GEMMs are tunable for experiments
-        const char* es = getenv("FSB_STAGES");
-        const char* ec = getenv("FSB_CTAS_PER_SM");
-        h->step_stages = es ? atoi(es) : 4;
-        const int per_sm = ec ? std::max(1, std::min(2, atoi(ec))) : 2;
-        h->step_ctas = h->num_sms * per_sm;
-    }
+    h->step_ctas = h->num_sms * kStepCtasPerSm;
 
     auto B16 = [](const void* p) { return reinterpret_cast<const bf16*>(p); };
     h->emb = B16(w->d_embeddings);
@@ -800,10 +786,7 @@ int fsb_lm_bench_gemms(fsb_lm* h, int reps, double* weight_bytes_per_rep, int* l
     auto run = [&](const StepGemmPlan& p) -> int {
         bytes += p.weight_bytes;
         ++launches;
-        StepGemmPlan q = p;
-        q.p.rows = rows;
-        FSB_TRY(step_finalize_launch(q, st));
-        return step_gemm_launch(q, st);
+        return launch_step(h, p, rows, st);
     };
     for (int r = 0; r < reps; ++r) {
         bytes = 0;

@@ -7,8 +7,6 @@
 #include "lm_gemm.cuh"
 #include "umma.cuh"
 
-#include <stdlib.h>
-
 #include <algorithm>
 #include <vector>
 
@@ -23,14 +21,12 @@ constexpr int kTmemCols = 2 * kBN;  // two accumulators: the stores of item n ov
 constexpr int kEpiThreads = 128;
 constexpr int kLoaderThreads = 128;  // four normaliser warps: two 16-byte cells per thread and k-block
 constexpr int kScratchBytes = 1024;  // r_s[32] | red[4][32]
+// batch rows per finalize unit (measured best): one load round per unit (<= 4 / <= 16 partials), every unit on its own CTA
+constexpr int kSwigluRowBlock = 8;
+constexpr int kResidRowBlock = 2;
 
 __device__ __forceinline__ void bar_sync(int id, int n) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory");
-}
-__device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
 }
 
 // ---- step_finalize: one unit = rows [j0, j0 + R) x the 128 features of tile `tile` of the PREVIOUS GEMM's output;
@@ -52,7 +48,7 @@ __device__ __forceinline__ void rows_warp_sums(const float (&sq)[R], float* red,
 template <int R, int UQ>  // UQ = partials fetched per round
 __device__ __forceinline__ void prev_sums(const StepGemmParams& p, int tile, int tid, int j0, float (&acc)[R]) {
     const int np = __ldg(p.prev.nparts + tile);
-    const int maxp = p.prev.max_parts;  // loads are bounded by the launch constant, see step_partial_sum
+    const int maxp = p.prev.max_parts;  // loads are bounded by the launch constant, see step_partial_sums
 #pragma unroll
     for (int r = 0; r < R; ++r) acc[r] = 0.f;
     const float* src = p.prev.ws + (static_cast<size_t>(tile) * 32 + j0) * 128 + tid;
@@ -177,12 +173,7 @@ step_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int item_begin = p.cta_items[blockIdx.x], item_end = p.cta_items[blockIdx.x + 1];
     unsigned long long* trace = p.trace ? p.trace + static_cast<size_t>(blockIdx.x) * 8 : nullptr;
-    if (trace && threadIdx.x == 0) {
-        unsigned smid;
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        trace[0] = globaltimer_ns();
-        (void)smid;
-    }
+    if (trace && threadIdx.x == 0) trace[0] = globaltimer_ns();
 
     if (warp == 4 && lane == 0) {
         tma_prefetch_desc(&tmA);
@@ -224,17 +215,6 @@ step_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                     tma_load_3d(tiles + static_cast<uint32_t>(s) * kStageBytes, &tmA, full0 + 8u * s, kb * kBlockK,
                                 w.x * kBlockM, 0, p.a_hint);
                     ++pre;
-                    if (++kb >= w.z) {
-                        if (++n < item_end) {
-                            w = p.sched[n];
-                            kb = w.y;
-                        }
-                    }
-                }
-                // ... optionally (FSB_L2_PREFETCH, default 0: measured no gain, profiles/r02_l2_prefetch.md) the weight
-                // tiles after those are requested into L2
-                for (int q = 0; q < p.l2_prefetch && n < item_end; ++q) {
-                    tma_prefetch_l2_3d(&tmA, kb * kBlockK, w.x * kBlockM, 0);
                     if (++kb >= w.z) {
                         if (++n < item_end) {
                             w = p.sched[n];
@@ -508,10 +488,6 @@ int step_plan_init(StepGemmPlan* plan, const __nv_bfloat16* w, int n_out, int K,
     p.b_hint = kEvictLast;   // the activation tile is re-read by every CTA
     p.ws = ws;
     p.prev_rb = 32;
-    {
-        const char* e = getenv("FSB_L2_PREFETCH");
-        p.l2_prefetch = e ? atoi(e) : 0;  // k-blocks per CTA (16 KB each); measured: no gain on B200 (profiles/)
-    }
     plan->grid = dim3(static_cast<unsigned>(num_ctas), 1, 1);
     plan->smem = smem_of(stages);
     plan->pro = PRO_NONE;
@@ -549,10 +525,7 @@ int step_finalize_launch(const StepGemmPlan& consumer, cudaStream_t st, int rb) 
     const int pro = consumer.pro;
     if (pro == PRO_NONE) return 0;
     StepGemmParams p = consumer.p;
-    // one load round per unit (<= 4 / <= 16 partials), every unit on its own CTA
-    static const int rb_swiglu = [] { const char* e = getenv("FSB_SWIGLU_RB"); return e ? atoi(e) : 8; }();
-    static const int rb_resid = [] { const char* e = getenv("FSB_RESID_RB"); return e ? atoi(e) : 2; }();
-    if (rb <= 0) rb = pro == PRO_SWIGLU ? rb_swiglu : rb_resid;
+    if (rb <= 0) rb = pro == PRO_SWIGLU ? kSwigluRowBlock : kResidRowBlock;
     FSB_CHECK(rb >= 1 && rb <= 32 && (rb & (rb - 1)) == 0, "finalize: row block %d is not a power of two <= 32", rb);
     p.prev_rb = rb;
     const int units = p.prev.tiles * cdiv(p.rows, rb);

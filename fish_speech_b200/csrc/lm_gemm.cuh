@@ -47,27 +47,10 @@ struct StepPartials {
 };
 
 #ifdef __CUDACC__
-// one output element, partials added in slot order
-__device__ __forceinline__ float step_partial_sum(const StepPartials& P, int row, int feat) {
-    const int tile = feat >> 7;
-    const int np = __ldg(P.nparts + tile);
-    const float* p = P.ws + (static_cast<size_t>(tile) * 32 + row) * 128 + (feat & 127);
-    const size_t ss = static_cast<size_t>(P.tiles) * 32 * 128;
-    float s = 0.f;
-    // The loads are bounded by max_parts (a launch constant), not by this tile's count: they leave together with
-    // the load of the count instead of one round trip behind it; slots >= np hold stale data and are not added.
-    for (int q = 0; q < P.max_parts; q += 8) {  // eight loads in flight, additions in slot order
-        float a[8];
-#pragma unroll
-        for (int u = 0; u < 8; ++u) a[u] = q + u < P.max_parts ? __ldcg(p + static_cast<size_t>(q + u) * ss) : 0.f;
-#pragma unroll
-        for (int u = 0; u < 8; ++u)
-            if (q + u < np) s += a[u];
-    }
-    return s;
-}
-// N output elements of one row at once: all loads of an 8-slot round are in flight together (N * 8 requests), the
-// additions stay in slot order -- bitwise the same sums as step_partial_sum.
+// N output elements of one row at once, partials added in slot order: all loads of an 8-slot round are in flight
+// together (N * 8 requests).  The loads are bounded by max_parts (a launch constant), not by each tile's count: they
+// leave together with the load of the count instead of one round trip behind it; slots >= np hold stale data and are
+// not added.
 template <int N>
 __device__ __forceinline__ void step_partial_sums(const StepPartials& P, int row, const int (&feat)[N], const bool (&ok)[N],
                                                   float (&out)[N]) {
@@ -81,7 +64,7 @@ __device__ __forceinline__ void step_partial_sums(const StepPartials& P, int row
         p[k] = P.ws + (static_cast<size_t>(f >> 7) * 32 + row) * 128 + (f & 127);
         out[k] = 0.f;
     }
-    for (int q = 0; q < P.max_parts; q += 8) {  // bounded by the launch constant: see step_partial_sum
+    for (int q = 0; q < P.max_parts; q += 8) {
         float a[N][8];
 #pragma unroll
         for (int k = 0; k < N; ++k)
@@ -104,7 +87,6 @@ struct StepGemmParams {
     int tiles, stages;
     int n_out, K;           // output features, reduction length
     int rows;               // live batch rows (<= 32)
-    int l2_prefetch;        // weight k-blocks per CTA prefetched into L2 behind the ring, before the operand exists
     unsigned long long a_hint, b_hint;
     float* ws;              // out: [slot][tile][32 rows][128 features] fp32 partials
     // ---- step_finalize of the GEMM that produces this one's operand (pro != PRO_NONE) ----
@@ -151,7 +133,7 @@ void step_plan_set_prev(StepGemmPlan* plan, int pro, const StepGemmPlan& prev);
 void step_plan_free(StepGemmPlan* plan);
 int step_gemm_launch(const StepGemmPlan& plan, cudaStream_t stream);
 // finish the GEMM that produces `consumer`'s operand (no-op when consumer.pro == PRO_NONE); launch it before the consumer.
-// rb: batch rows per finalize unit (power of two <= 32); 0 = FSB_SWIGLU_RB / FSB_RESID_RB or the default (8 / 2)
+// rb: batch rows per finalize unit (power of two <= 32); 0 = the measured best (8 for SwiGLU, 2 for the residual add)
 int step_finalize_launch(const StepGemmPlan& consumer, cudaStream_t stream, int rb = 0);
 int step_gemm_init();  // kernel attributes (idempotent)
 

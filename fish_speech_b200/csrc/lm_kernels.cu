@@ -117,58 +117,19 @@ __global__ void __launch_bounds__(kRowThreads) rows_kernel(RowsArgs a) {
 // ------------------------------------------------------------------------------------------------
 // residual add + fish RMSNorm on a plain fp32 GEMM result (prefill, codec transformer)
 // ------------------------------------------------------------------------------------------------
-constexpr int kRnThreads = 512;
-constexpr int kRnMaxPer = 8;  // D <= 4096
-
+// 4 consecutive features per thread (D % 4 == 0, ld % 4 == 0): 16-byte loads of y.
+constexpr int kRnThreads = 256;
+constexpr int kRnMaxPer = 4;  // D <= 4096
 __global__ void __launch_bounds__(kRnThreads) resid_norm_kernel(ResidNormArgs a) {
     pdl_launch_dependents();
     pdl_wait();
     __shared__ float red[33];
     const int row = blockIdx.x;
-    float v[kRnMaxPer];
+    float v[kRnMaxPer][4];
     float ss = 0.f;
 #pragma unroll
     for (int e = 0; e < kRnMaxPer; ++e) {
-        const int f = threadIdx.x + e * kRnThreads;
-        v[e] = 0.f;
-        if (f < a.D) {
-            float x = a.x_in ? bf2f(a.x_in[static_cast<size_t>(row) * a.D + f]) : 0.f;
-            if (a.y) {
-                float yy = a.y[static_cast<size_t>(row) * a.ld + f];
-                if (a.bias) yy += bf2f(a.bias[f]);
-                yy = rbf(yy);
-                if (a.scale) yy *= bf2f(a.scale[f]);
-                x = rbf(x + yy);
-            }
-            v[e] = x;
-            ss += x * x;
-            if (a.x_out) a.x_out[static_cast<size_t>(row) * a.D + f] = f2bf(x);
-        }
-    }
-    if (a.norm_w != nullptr) {
-        const float tot = block_sum(ss, red);
-        const float r = rsqrtf(tot / static_cast<float>(a.D) + a.eps);
-#pragma unroll
-        for (int e = 0; e < kRnMaxPer; ++e) {
-            const int f = threadIdx.x + e * kRnThreads;
-            if (f < a.D) a.n_out[static_cast<size_t>(row) * a.D + f] = f2bf(rbf(rbf(v[e] * r) * bf2f(a.norm_w[f])));
-        }
-    }
-}
-
-// Vectorised form (D % 4 == 0, ld % 4 == 0): 4 consecutive features per thread, 16-byte loads of y.
-constexpr int kRn4Threads = 256;
-constexpr int kRn4MaxPer = 4;  // D <= 4096
-__global__ void __launch_bounds__(kRn4Threads) resid_norm4_kernel(ResidNormArgs a) {
-    pdl_launch_dependents();
-    pdl_wait();
-    __shared__ float red[33];
-    const int row = blockIdx.x;
-    float v[kRn4MaxPer][4];
-    float ss = 0.f;
-#pragma unroll
-    for (int e = 0; e < kRn4MaxPer; ++e) {
-        const int f = (threadIdx.x + e * kRn4Threads) * 4;
+        const int f = (threadIdx.x + e * kRnThreads) * 4;
         v[e][0] = v[e][1] = v[e][2] = v[e][3] = 0.f;
         if (f >= a.D) continue;
         float x[4] = {0.f, 0.f, 0.f, 0.f};
@@ -208,8 +169,8 @@ __global__ void __launch_bounds__(kRn4Threads) resid_norm4_kernel(ResidNormArgs 
         const float tot = block_sum(ss, red);
         const float r = rsqrtf(tot / static_cast<float>(a.D) + a.eps);
 #pragma unroll
-        for (int e = 0; e < kRn4MaxPer; ++e) {
-            const int f = (threadIdx.x + e * kRn4Threads) * 4;
+        for (int e = 0; e < kRnMaxPer; ++e) {
+            const int f = (threadIdx.x + e * kRnThreads) * 4;
             if (f >= a.D) continue;
             const uint2 w = *reinterpret_cast<const uint2*>(a.norm_w + f);
             const float wf[4] = {bf_lo(w.x), bf_hi(w.x), bf_lo(w.y), bf_hi(w.y)};
@@ -227,60 +188,11 @@ __global__ void __launch_bounds__(kRn4Threads) resid_norm4_kernel(ResidNormArgs 
 // ------------------------------------------------------------------------------------------------
 // q/k/v post-processing: llama.py:891-911
 // ------------------------------------------------------------------------------------------------
-__global__ void qkv_prep_kernel(QkvPrepArgs a) {
-    pdl_launch_dependents();
-    pdl_wait();
-    __shared__ float red[33];
-    const int row = blockIdx.x, head = blockIdx.y;
-    const int t = threadIdx.x;  // pair index, Dh/2 threads
-    const int Dh = a.Dh;
-    const int kind = head < a.H ? 0 : (head < a.H + a.Hkv ? 1 : 2);  // q, k, v
-    const int f0 = head * Dh + 2 * t;
-    const float2 y2 = *reinterpret_cast<const float2*>(a.y + static_cast<size_t>(row) * a.ld + f0);
-    float v0 = y2.x, v1 = y2.y;
-    if (a.bias) {
-        v0 += bf2f(a.bias[f0]);
-        v1 += bf2f(a.bias[f0 + 1]);
-    }
-    v0 = rbf(v0);
-    v1 = rbf(v1);
-    const __nv_bfloat16* nw = kind == 0 ? a.q_norm : (kind == 1 ? a.k_norm : nullptr);
-    if (nw != nullptr) {
-        // nn.RMSNorm(head_dim): fp32 math, weight multiply included, ONE rounding
-        const float tot = block_sum(v0 * v0 + v1 * v1, red);
-        const float r = rsqrtf(tot / static_cast<float>(Dh) + a.eps);
-        v0 = rbf(v0 * r * bf2f(nw[2 * t]));
-        v1 = rbf(v1 * r * bf2f(nw[2 * t + 1]));
-    }
-    const int pos = a.row_pos[row];
-    if (kind != 2) {
-        const __nv_bfloat16* f = a.freqs + (static_cast<size_t>(max(pos, 0)) * (Dh / 2) + t) * 2;
-        const float c = bf2f(f[0]), s = bf2f(f[1]);
-        const float o0 = __fsub_rn(__fmul_rn(v0, c), __fmul_rn(v1, s));
-        const float o1 = __fadd_rn(__fmul_rn(v1, c), __fmul_rn(v0, s));
-        v0 = rbf(o0);
-        v1 = rbf(o1);
-    }
-    const uint32_t packed = pack_bf2(v0, v1);
-    if (kind == 0) {
-        uint32_t* dst = reinterpret_cast<uint32_t*>(a.q + (static_cast<size_t>(row) * a.H + head) * Dh);
-        dst[t] = packed;
-    } else if (pos >= 0 && pos < a.S) {
-        const int g = kind == 1 ? head - a.H : head - a.H - a.Hkv;
-        __nv_bfloat16* cache = kind == 1 ? a.kcache : a.vcache;
-        const int b = a.row_seq[row];
-        uint32_t* dst = reinterpret_cast<uint32_t*>(
-            cache + ((static_cast<size_t>(b) * a.Hkv + g) * a.S + pos) * Dh);
-        dst[t] = packed;
-    }
-}
-
-// The same per (row, head) work with one CTA per row: a warp takes whole heads (lane = rotary pair, two pairs per lane
-// at head_dim 128), so the per-head norm is a warp reduction and a row costs one CTA of 8 warps instead of H + 2 Hkv
-// CTAs of Dh / 2 threads (393 216 one-warp CTAs per codec transformer layer at 32 x 256 frames).
-constexpr int kQkvRowThreads = 256;
+// One CTA per row: a warp takes whole heads (lane = rotary pair, two pairs per lane at head_dim 128), so the per-head
+// norm is a warp reduction.
+constexpr int kQkvThreads = 256;
 template <int DH>
-__global__ void __launch_bounds__(kQkvRowThreads) qkv_prep_row_kernel(QkvPrepArgs a) {
+__global__ void __launch_bounds__(kQkvThreads) qkv_prep_kernel(QkvPrepArgs a) {
     pdl_launch_dependents();
     pdl_wait();
     constexpr int PPL = DH / 64;  // rotary pairs per lane
@@ -289,7 +201,7 @@ __global__ void __launch_bounds__(kQkvRowThreads) qkv_prep_row_kernel(QkvPrepArg
     const int pos = a.row_pos[row];
     const int b = a.row_seq[row];
     const int NH = a.H + 2 * a.Hkv;
-    for (int head = warp; head < NH; head += kQkvRowThreads / 32) {
+    for (int head = warp; head < NH; head += kQkvThreads / 32) {
         const int kind = head < a.H ? 0 : (head < a.H + a.Hkv ? 1 : 2);  // q, k, v
         const __nv_bfloat16* nw = kind == 0 ? a.q_norm : (kind == 1 ? a.k_norm : nullptr);
         float v0[PPL], v1[PPL];
@@ -509,38 +421,6 @@ __device__ __forceinline__ void attend(const float* qs, float* sc, float* red, c
 }
 
 
-template <int DH, int G>
-__global__ void __launch_bounds__(kAttnThreads) attn_kernel(AttnArgs a, float scale, int lcap) {
-    pdl_launch_dependents();
-    pdl_wait();
-    extern __shared__ float sm[];
-    float* qs = sm;                      // [G][DH]
-    float* sc = qs + G * DH;             // [G][lcap]
-    float* red = sc + G * lcap;          // [kAttnWarps][G][DH]
-    const int row = blockIdx.y, g = blockIdx.x;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int b = a.row_seq[row], pos = min(a.row_pos[row], a.S - 1);  // a position past the cache reads its last row
-    if (pos < 0) {  // idle slot parked at position -1: nothing to attend to
-        for (int e = threadIdx.x; e < G * DH; e += kAttnThreads)
-            a.out[(static_cast<size_t>(row) * a.H + blockIdx.x * G) * DH + e] = f2bf(0.f);
-        return;
-    }
-    const int lo = (a.window > 0 && pos - a.window + 1 > 0) ? pos - a.window + 1 : 0;
-    const int L = pos - lo + 1;
-    const size_t cache_base = ((static_cast<size_t>(b) * a.Hkv + g) * a.S + lo) * DH;
-    const __nv_bfloat16* kc = a.kcache + cache_base;
-    const __nv_bfloat16* vc = a.vcache + cache_base;
-
-    for (int e = threadIdx.x; e < G * DH; e += kAttnThreads) {
-        const int gg = e / DH, d = e - gg * DH;
-        qs[e] = bf2f(a.q[(static_cast<size_t>(row) * a.H + g * G + gg) * DH + d]);
-    }
-    __syncthreads();
-
-    attend<DH, G>(qs, sc, red, kc, vc, L, lcap, scale, a.bf16_math,
-                  a.out + (static_cast<size_t>(row) * a.H + g * G) * DH);
-}
-
 // ------------------------------------------------------------------------------------------------
 // decode-step attention with the qkv GEMM's fix-up in front (see lm_kernels.cuh)
 // ------------------------------------------------------------------------------------------------
@@ -678,23 +558,9 @@ __global__ void __launch_bounds__(kAttnThreads) attn_decode_kernel(AttnDecodeArg
 }
 
 // ------------------------------------------------------------------------------------------------
-// SwiGLU on a plain fp32 GEMM result (prefill, codec): 4 consecutive features per thread where aligned
+// SwiGLU on a plain fp32 GEMM result (prefill, codec): 4 consecutive features per thread (I % 4 == 0, ld % 4 == 0)
 // ------------------------------------------------------------------------------------------------
 __global__ void swiglu_kernel(SwigluArgs a) {
-    pdl_launch_dependents();
-    pdl_wait();
-    const int row = blockIdx.y;
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= a.I) return;
-    const float* y = a.y + static_cast<size_t>(row) * a.ld;
-    const int gi = a.interleaved ? w13_gate_row(i) : i;
-    const int ui = a.interleaved ? gi + 16 : a.I + i;
-    const float g = rbf(y[gi]), c = rbf(y[ui]);
-    const float s = rbf(g / (1.f + expf(-g)));
-    a.h[static_cast<size_t>(row) * a.I + i] = f2bf(s * c);
-}
-
-__global__ void swiglu4_kernel(SwigluArgs a) {
     pdl_launch_dependents();
     pdl_wait();
     const int row = blockIdx.y;
@@ -1009,29 +875,26 @@ int launch_rows(const RowsArgs& a, cudaStream_t st) {
 
 int launch_resid_norm(const ResidNormArgs& a, cudaStream_t st) {
     if (a.rows <= 0) return 0;
-    FSB_CHECK(a.D <= kRnThreads * kRnMaxPer, "resid_norm: D=%d too large", a.D);
-    const bool vec = (a.D & 3) == 0 && (a.y == nullptr || ((a.ld & 3) == 0 && (reinterpret_cast<uintptr_t>(a.y) & 15) == 0));
-    if (vec) FSB_LAUNCH(resid_norm4_kernel, dim3(a.rows), dim3(kRn4Threads), 0, st, a);
-    else FSB_LAUNCH(resid_norm_kernel, dim3(a.rows), dim3(kRnThreads), 0, st, a);
+    FSB_CHECK(a.D % 4 == 0 && a.D <= 4 * kRnThreads * kRnMaxPer, "resid_norm: D=%d unsupported", a.D);
+    FSB_CHECK(a.y == nullptr || (a.ld % 4 == 0 && (reinterpret_cast<uintptr_t>(a.y) & 15) == 0),
+              "resid_norm: misaligned GEMM result");
+    FSB_LAUNCH(resid_norm_kernel, dim3(a.rows), dim3(kRnThreads), 0, st, a);
     return 0;
 }
 
 int launch_qkv_prep(const QkvPrepArgs& a, cudaStream_t st) {
     if (a.rows <= 0) return 0;
-    FSB_CHECK(a.Dh % 64 == 0 && a.Dh <= 256, "qkv_prep: head_dim %d unsupported", a.Dh);
+    FSB_CHECK(a.Dh == 64 || a.Dh == 128, "qkv_prep: head_dim %d unsupported", a.Dh);
     FSB_CHECK((a.ld & 1) == 0 && (reinterpret_cast<uintptr_t>(a.y) & 7) == 0, "qkv_prep: misaligned GEMM result");
-    if (a.Dh == 64) FSB_LAUNCH(qkv_prep_row_kernel<64>, dim3(a.rows), dim3(kQkvRowThreads), 0, st, a);
-    else if (a.Dh == 128) FSB_LAUNCH(qkv_prep_row_kernel<128>, dim3(a.rows), dim3(kQkvRowThreads), 0, st, a);
-    else FSB_LAUNCH(qkv_prep_kernel, dim3(a.rows, a.H + 2 * a.Hkv), dim3(a.Dh / 2), 0, st, a);
+    if (a.Dh == 64) FSB_LAUNCH(qkv_prep_kernel<64>, dim3(a.rows), dim3(kQkvThreads), 0, st, a);
+    else FSB_LAUNCH(qkv_prep_kernel<128>, dim3(a.rows), dim3(kQkvThreads), 0, st, a);
     return 0;
 }
 
 // Score-buffer positions per head for a context bound of `need`: rounded up to a multiple of 32 and cut to what fits
 // 200 KB of shared memory (a longer context is walked in chunks, see attend()).  g_attn_chunk (tests) forces a chunk.
 static int g_attn_chunk = 0;
-static bool g_attn_per_row = false;  // tests: launch_attn uses the per-row kernel (the decode kernel's attention core)
 void attn_set_score_chunk(int positions) { g_attn_chunk = positions > 0 ? (positions + 31) / 32 * 32 : 0; }
-void attn_force_per_row(bool on) { g_attn_per_row = on; }
 template <int DH, int G>
 static size_t attn_smem_bytes(int lcap) {
     return (static_cast<size_t>(G) * DH + static_cast<size_t>(G) * lcap + static_cast<size_t>(kAttnWarps) * G * DH) *
@@ -1046,22 +909,10 @@ static int attn_score_chunk(int need) {
     return lcap;
 }
 
-template <int DH, int G>
-static int launch_attn_t(const AttnArgs& a, cudaStream_t st) {
-    int lcap = a.window > 0 && a.window < a.S ? a.window : a.S;
-    if (a.lcap > 0 && a.lcap < lcap) lcap = a.lcap;
-    lcap = attn_score_chunk<DH, G>(lcap);
-    const size_t smem = attn_smem_bytes<DH, G>(lcap);
-    const float scale = 1.0f / sqrtf(static_cast<float>(DH));
-    FSB_LAUNCH((attn_kernel<DH, G>), dim3(a.Hkv, a.rows), dim3(kAttnThreads), smem, st, a, scale, lcap);
-    return 0;
-}
-
 int attn_init() {
     static bool done = false;
     if (done) return 0;
 #define FSB_ATTN_ATTR(DH_, G_) \
-    FSB_CUDA(cudaFuncSetAttribute(attn_kernel<DH_, G_>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024)); \
     FSB_CUDA(cudaFuncSetAttribute(attn_decode_kernel<DH_, G_>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     FSB_ATTN_ATTR(128, 1) FSB_ATTN_ATTR(128, 2) FSB_ATTN_ATTR(128, 4) FSB_ATTN_ATTR(128, 8)
     FSB_ATTN_ATTR(64, 1) FSB_ATTN_ATTR(64, 2) FSB_ATTN_ATTR(64, 4) FSB_ATTN_ATTR(64, 8)
@@ -1094,27 +945,11 @@ int launch_attn_decode(const AttnDecodeArgs& a, cudaStream_t st) {
     return 1;
 }
 
-int launch_attn(const AttnArgs& a, cudaStream_t st) {
-    if (a.rows <= 0) return 0;
-    // one kernel whatever the number of rows: a sequence must get the same bits alone, in a batch or in pieces
-    static const bool tile_on = [] { const char* e = getenv("FSB_ATTN_TILE"); return !(e && e[0] == '0'); }();
-    if (tile_on && !g_attn_per_row && attn_tile_supported(a)) return launch_attn_tile(a, st);
-    const int G = a.H / a.Hkv;
-    FSB_CHECK(a.H % a.Hkv == 0, "attention: H %% Hkv != 0");
-#define FSB_ATTN_CASE(DH_, G_) \
-    if (a.Dh == DH_ && G == G_) return launch_attn_t<DH_, G_>(a, st);
-    FSB_ATTN_CASE(128, 1) FSB_ATTN_CASE(128, 2) FSB_ATTN_CASE(128, 4) FSB_ATTN_CASE(128, 8)
-    FSB_ATTN_CASE(64, 1) FSB_ATTN_CASE(64, 2) FSB_ATTN_CASE(64, 4) FSB_ATTN_CASE(64, 8)
-#undef FSB_ATTN_CASE
-    set_error("attention: unsupported head_dim=%d group=%d", a.Dh, G);
-    return 1;
-}
-
 int launch_swiglu(const SwigluArgs& a, cudaStream_t st) {
     if (a.rows <= 0) return 0;
-    const bool vec = (a.I & 3) == 0 && (a.ld & 3) == 0 && (reinterpret_cast<uintptr_t>(a.y) & 15) == 0;
-    if (vec) FSB_LAUNCH(swiglu4_kernel, dim3(cdiv(a.I, 1024), a.rows), dim3(256), 0, st, a);
-    else FSB_LAUNCH(swiglu_kernel, dim3(cdiv(a.I, 256), a.rows), dim3(256), 0, st, a);
+    FSB_CHECK(a.I % 4 == 0, "swiglu: I=%d unsupported", a.I);
+    FSB_CHECK(a.ld % 4 == 0 && (reinterpret_cast<uintptr_t>(a.y) & 15) == 0, "swiglu: misaligned GEMM result");
+    FSB_LAUNCH(swiglu_kernel, dim3(cdiv(a.I, 1024), a.rows), dim3(256), 0, st, a);
     return 0;
 }
 

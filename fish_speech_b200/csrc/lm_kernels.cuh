@@ -78,9 +78,7 @@ struct QkvPrepArgs {
 };
 int launch_qkv_prep(const QkvPrepArgs& a, cudaStream_t st);
 
-// out[row][h][:] = softmax(q.k^T * scale over cache positions [max(0,pos-window+1), pos]) . v
-// bf16_math = 1 reproduces the fast-AR hand-rolled attention (llama.py:948-976): scores, scaled
-// scores, probabilities and the output are each rounded to bf16.
+// out[row][h][:] = softmax(q.k^T * scale over cache positions [max(0,pos-window+1), pos]) . v  (fp32 softmax)
 struct AttnArgs {
     const __nv_bfloat16* q;  // [rows, H, Dh]
     const __nv_bfloat16* kcache;
@@ -90,17 +88,12 @@ struct AttnArgs {
     __nv_bfloat16* out;  // [rows, H*Dh]
     int rows, H, Hkv, Dh, S;
     int window;  // <=0: unlimited
-    int lcap;    // score-buffer length: an upper bound of (row_pos + 1); 0 = cache capacity S
-    int bf16_math;
 };
+// csrc/attn_tile.cu: 64 rows of one head per CTA, K/V tiles staged once, mma.sync tensor cores, online softmax; for any
+// number of rows (prefill, codec transformer).  head_dim 64 or 128.
 int launch_attn(const AttnArgs& a, cudaStream_t st);
-// csrc/attn_tile.cu: 64 rows of one head per CTA, K/V tiles staged once, mma.sync tensor cores, online softmax; what
-// launch_attn uses for >= 64 rows (prefill, codec transformer).  FSB_ATTN_TILE=0 keeps the per-row kernel.
-bool attn_tile_supported(const AttnArgs& a);
-int launch_attn_tile(const AttnArgs& a, cudaStream_t st);
-int attn_init();  // set kernel attributes (idempotent)
-void attn_set_score_chunk(int positions);  // tests: force the score-buffer chunk (0 = automatic)
-void attn_force_per_row(bool on);          // tests: launch_attn runs the per-row kernel instead of the tiled one
+int attn_init();  // set the decode attention's kernel attributes (idempotent)
+void attn_set_score_chunk(int positions);  // tests: force the decode attention's score-buffer chunk (0 = automatic)
 
 // Decode-step attention: the consumer of the qkv step GEMM. One CTA per (batch row, KV group) first finishes that
 // GEMM for its own (G + 2) heads -- slot-ordered sum of the stream-K partials, bias, per-head nn.RMSNorm, interleaved

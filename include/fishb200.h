@@ -278,12 +278,10 @@ int fsb_op_attn_decode(const float* d_ws, const int32_t* d_nparts, int tiles, in
                        const int32_t* d_row_seq, const int32_t* d_row_pos, void* d_out, int rows, int H, int Hkv,
                        int Dh, int S, int lcap, int bf16_math, int kv_only, float eps, void* stream);
 
-/* Attention keeps one fp32 score per position and head in shared memory; contexts longer than the buffer are walked
- * in chunks, bit-identically (csrc/lm_kernels.cu attend()).  positions > 0 forces a smaller chunk; 0 = automatic. */
+/* The decode attention (fsb_op_attn_decode, the decode frame) keeps one fp32 score per position and head in shared
+ * memory; contexts longer than the buffer are walked in chunks, bit-identically (csrc/lm_kernels.cu attend()).
+ * positions > 0 forces a smaller chunk; 0 = automatic. */
 int fsb_op_attn_score_chunk(int positions);
-/* fsb_window_attn normally runs the tiled tensor-core kernel (csrc/attn_tile.cu); on != 0 makes it run the per-row
- * kernel, whose attention core is the one of the decode step (what the chunking test above exercises). */
-int fsb_op_attn_per_row(int on);
 /* Diagnostics of fsb_res_unit: d_trace [64][6] globaltimer stamps of CTA 0's first tiles = {epilogue idle, conv7
  * accumulator ready, h written, conv1 accumulator ready, outputs staged, stores issued}; NULL switches it off. */
 int fsb_op_res_unit_trace(unsigned long long* d_trace);

@@ -161,45 +161,6 @@ def test_conv_gemm_causal_dilated_and_transposed():
     assert err <= 2e-2 * max(1.0, ref.abs().max().item()), err
 
 
-@pytest.mark.parametrize("H,Hkv,Dh", [(8, 2, 128), (4, 4, 64)])
-def test_attention_past_the_score_buffer_is_chunked_bit_identically(H, Hkv, Dh):
-    """Contexts longer than the shared-memory score buffer (~12.5 k positions at G=4) are walked in chunks: same bits
-    whatever the chunk (forced to 64 / 4096 positions here), and the fp32 SDPA answer (llama.py:916-934) at 20 000."""
-    _l, L = _lib()
-    S = 20000
-    g = torch.Generator().manual_seed(S + H)
-    k = (torch.randn(1, Hkv, S, Dh, generator=g)).bfloat16()
-    v = (torch.randn(1, Hkv, S, Dh, generator=g)).bfloat16()
-    pos = torch.tensor([0, 31, 32, 63, 64, 4095, 4096, 12543, 12544, 17001, S - 1], dtype=torch.int32)
-    rows = pos.numel()
-    q = (torch.randn(rows, H, Dh, generator=g) * 1.5).bfloat16()
-    seq = torch.zeros(rows, dtype=torch.int32)
-    dq, dk, dv, dseq, dpos = q.cuda(), k.cuda(), v.cuda(), seq.cuda(), pos.cuda()
-
-    def run(chunk):
-        _l.check(L.fsb_op_attn_score_chunk(chunk))
-        _l.check(L.fsb_op_attn_per_row(1))  # the per-row kernel = the decode step's attention core
-        out = torch.empty(rows, H * Dh, dtype=torch.bfloat16, device="cuda")
-        try:
-            _l.check(L.fsb_window_attn(dq.data_ptr(), dk.data_ptr(), dv.data_ptr(), dseq.data_ptr(), dpos.data_ptr(), rows,
-                                       H, Hkv, Dh, S, 0, out.data_ptr(), _st()))
-            torch.cuda.synchronize()
-        finally:
-            L.fsb_op_attn_score_chunk(0)
-            L.fsb_op_attn_per_row(0)
-        return out.cpu()
-
-    auto = run(0)
-    assert torch.equal(run(64), auto) and torch.equal(run(4096), auto)
-    kk = k[0].float().repeat_interleave(H // Hkv, dim=0)  # [H,S,Dh]
-    vv = v[0].float().repeat_interleave(H // Hkv, dim=0)
-    for i, p in enumerate(pos.tolist()):
-        s = torch.einsum("hd,hsd->hs", q[i].float(), kk[:, :p + 1]) / Dh ** 0.5
-        ref = torch.einsum("hs,hsd->hd", torch.softmax(s, -1), vv[:, :p + 1]).reshape(-1)
-        err = (auto[i].float() - ref).abs().max().item()
-        assert err <= 2 ** -7 * ref.abs().max().item() + 1e-3, (p, err)
-
-
 @pytest.mark.parametrize("C,dil,B,T", [(96, 1, 2, 300), (192, 3, 1, 517), (192, 9, 2, 128), (384, 9, 2, 260), (96, 9, 1, 40)])
 def test_fused_residual_unit_equals_two_conv_launches(C, dil, B, T):
     """csrc/codec_resunit.cu (Snake -> dilated conv7 -> Snake -> conv1 -> + x in one kernel, the intermediate in shared

@@ -546,3 +546,60 @@ def test_attn_decode(Dh, G, bias, qk_norm, bf16_math):
     assert torch.equal(bits(kc2), bits(kc)) and torch.equal(bits(out2), bits(out)), "chunked attention differs"
     print(f"\nattn_decode Dh={Dh} G={G} bias={bias} qk_norm={qk_norm} bf16_math={bf16_math}: max_parts {maxp}, "
           f"worst err/bound {worst:.3f}, ambiguous {n_amb}")
+
+
+@pytest.mark.parametrize("H,Hkv,Dh", [(8, 2, 128), (4, 4, 64)])
+def test_attention_past_the_score_buffer_is_chunked_bit_identically(H, Hkv, Dh):
+    """Contexts longer than the shared-memory score buffer (11 648 positions at G=4, head_dim 128) are walked in chunks
+    by attend(): same bits whatever the chunk (forced to 64 / 4096 positions here), and the fp32 SDPA answer
+    (llama.py:916-934) at 20 000. Every row has its own KV slot holding the same history, since the kernel appends the
+    row's K/V at its position. q, k and v come as a one-slot partial set of bf16 values, without bias or qk-norm and
+    with a RoPE table of (cos, sin) = (1, 0): they reach the scores and the cache unchanged. A row's own key scores a
+    little above the history's maximum for almost every head, so the maximum sits in the last chunk of every walk;
+    the history still carries much of a long row's weight."""
+    _l, L = _lib()
+    S = 20000
+    G = H // Hkv
+    n_out = (H + 2 * Hkv) * Dh
+    tiles = cdiv(n_out, 128)
+    g = torch.Generator().manual_seed(S + H)
+    k = torch.randn(Hkv, S, Dh, generator=g).bfloat16()
+    v = torch.randn(Hkv, S, Dh, generator=g).bfloat16()
+    pos = torch.tensor([0, 31, 32, 63, 64, 4095, 4096, 12543, 12544, 17001, S - 1], dtype=torch.int32)
+    rows = pos.numel()
+    q = (torch.randn(rows, Hkv, G, Dh, generator=g) * 1.5).bfloat16().float()
+    k_new = q.sum(2)  # scaled so that q . k_new / sqrt(Dh) is 8 on average (the history's maximum is about 6)
+    k_new = (k_new * (8 * math.sqrt(Dh) / torch.einsum("rhgd,rhd->rhg", q, k_new).mean())).bfloat16().float()
+    v_new = torch.randn(rows, Hkv * Dh, generator=g).bfloat16().float()
+    qkv = torch.full((ROWS, tiles * 128), float("nan"))
+    qkv[:rows, :n_out] = torch.cat([q.reshape(rows, -1), k_new.reshape(rows, -1), v_new], 1)
+    ws = qkv.view(ROWS, tiles, 128).transpose(0, 1).contiguous()[None]  # slot 0 of [slots, tiles, 32, 128]
+    freqs = torch.zeros(S, Dh // 2, 2)
+    freqs[..., 0] = 1.0
+    dws, dnp = ws.cuda(), torch.ones(tiles, dtype=torch.int32, device="cuda")
+    dfr, dseq, dpos = freqs.bfloat16().cuda(), torch.arange(rows, dtype=torch.int32).cuda(), pos.cuda()
+    kc, vc = k.cuda()[None].repeat(rows, 1, 1, 1), v.cuda()[None].repeat(rows, 1, 1, 1)
+
+    def run(chunk):  # every run appends the same K/V at the same positions: the cache is the same for all of them
+        out = torch.full((rows, H * Dh), float("nan"), dtype=torch.bfloat16, device="cuda")
+        _l.check(L.fsb_op_attn_score_chunk(chunk))
+        try:
+            _l.check(L.fsb_op_attn_decode(dws.data_ptr(), dnp.data_ptr(), tiles, 1, None, None, None, dfr.data_ptr(),
+                                          kc.data_ptr(), vc.data_ptr(), dseq.data_ptr(), dpos.data_ptr(),
+                                          out.data_ptr(), rows, H, Hkv, Dh, S, 0, 0, 0, EPS, _st()))
+        finally:
+            L.fsb_op_attn_score_chunk(0)
+        return out.cpu()
+
+    auto = run(0)
+    assert torch.equal(bits(run(64)), bits(auto)) and torch.equal(bits(run(4096)), bits(auto))
+    scale = 1.0 / math.sqrt(Dh)
+    for i, p in enumerate(pos.tolist()):
+        K_, V_ = kc[i, :, : p + 1].cpu(), vc[i, :, : p + 1].cpu()  # the cache as the kernel left it
+        assert torch.equal(bits(K_[:, p]), bits(qkv[i, H * Dh : (H + Hkv) * Dh].bfloat16().view(Hkv, Dh)))
+        assert torch.equal(bits(V_[:, p]), bits(qkv[i, (H + Hkv) * Dh : n_out].bfloat16().view(Hkv, Dh)))
+        qi = qkv[i, : H * Dh].double().view(Hkv, G, Dh)
+        s = torch.einsum("hgd,hsd->hgs", qi, K_.double()) * scale
+        ref = torch.einsum("hgs,hsd->hgd", torch.softmax(s, -1), V_.double()).reshape(-1)
+        err = (auto[i].double() - ref).abs().max().item()
+        assert err <= 2 ** -7 * ref.abs().max().item() + 1e-3, (p, err)
