@@ -44,6 +44,25 @@ class Sampling(C.Structure):
                 ("seed", C.c_ulonglong)]
 
 
+class SlotCtlArgs(C.Structure):
+    """fsb_op_slot_ctl (include/fishb200.h)."""
+    _fields_ = [("state", C.c_void_p), ("limit", C.c_void_p), ("temperature", C.c_void_p), ("top_p", C.c_void_p),
+                ("top_k", C.c_void_p), ("seed", C.c_void_p), ("n_out", C.c_void_p)]
+
+
+class SampleArgs(C.Structure):
+    """fsb_op_sample_args (include/fishb200.h)."""
+    _fields_ = [("ws", C.c_void_p), ("nparts", C.c_void_p), ("tiles", C.c_int), ("max_parts", C.c_int),
+                ("n", C.c_int), ("rows", C.c_int), ("temperature", C.c_float), ("top_p", C.c_float),
+                ("top_k", C.c_int), ("slow", C.c_int), ("n_sem", C.c_int), ("sem_begin", C.c_int),
+                ("im_end_id", C.c_int), ("codebook_size", C.c_int), ("use_ras", C.c_int),
+                ("ras_window", C.c_void_p), ("ras_update", C.c_int), ("seed", C.c_ulonglong),
+                ("rng_offset", C.c_void_p), ("draw_id", C.c_int), ("cur_tok", C.c_void_p), ("cb_index", C.c_int),
+                ("num_cb", C.c_int), ("logits_out", C.c_void_p), ("finished", C.c_void_p),
+                ("row_slot", C.c_void_p), ("noise_u", C.c_void_p), ("noise_draws", C.c_int),
+                ("noise_ld", C.c_int), ("ctl", SlotCtlArgs)]
+
+
 _lib = None
 
 
@@ -109,6 +128,8 @@ def lib() -> C.CDLL:
     L.fsb_op_step_finalize.argtypes = [i32, vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, i32, vp]
     L.fsb_op_attn_decode.argtypes = [vp, vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32,
                                      i32, i32, i32, C.c_float, vp]
+    L.fsb_op_sample.argtypes = [C.POINTER(SampleArgs), vp]
+    L.fsb_op_frame_end.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, C.POINTER(SlotCtlArgs), vp]
     _lib = L
     return L
 

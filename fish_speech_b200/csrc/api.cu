@@ -194,4 +194,80 @@ int fsb_op_attn_decode(const float* d_ws, const int32_t* d_nparts, int tiles, in
     return 0;
 }
 
+static int hook_slot_ctl(const fsb_op_slot_ctl* c, SlotCtl* out) {
+    *out = SlotCtl{};
+    if (c == nullptr || c->state == nullptr) {
+        FSB_CHECK(c == nullptr || (!c->limit && !c->temperature && !c->top_p && !c->top_k && !c->seed && !c->n_out),
+                  "slot control without state");
+        return 0;
+    }
+    out->state = c->state;
+    out->limit = c->limit;
+    out->temperature = c->temperature;
+    out->top_p = c->top_p;
+    out->top_k = c->top_k;
+    out->seed = c->seed;
+    out->n_out = c->n_out;
+    return 0;
+}
+
+int fsb_op_sample(const fsb_op_sample_args* h, void* stream) {
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    FSB_CHECK(h->rows >= 1 && h->rows <= kStepRows && h->max_parts >= 1 && h->tiles == cdiv(h->n, 128),
+              "sample hook: shape");
+    SampleArgs a{};
+    FSB_TRY(hook_slot_ctl(&h->ctl, &a.ctl));
+    FSB_CHECK(!a.ctl.state || (a.ctl.limit && a.ctl.temperature && a.ctl.top_p && a.ctl.top_k && a.ctl.seed &&
+                               a.ctl.n_out),
+              "sample hook: slot control needs all seven arrays");
+    a.parts = hook_partials(h->ws, h->nparts, h->tiles, h->n, h->max_parts);
+    a.n = h->n;
+    a.rows = h->rows;
+    a.temperature = h->temperature; a.top_p = h->top_p; a.top_k = h->top_k;
+    a.slow = h->slow;
+    a.n_sem = h->n_sem; a.sem_begin = h->sem_begin; a.im_end_id = h->im_end_id; a.codebook_size = h->codebook_size;
+    a.use_ras = h->use_ras;
+    a.ras_window = h->ras_window;
+    a.ras_update = h->ras_update;
+    a.seed = h->seed;
+    a.rng_offset = h->rng_offset;
+    a.draw_id = h->draw_id;
+    a.cur_tok = h->cur_tok;
+    a.cb_index = h->cb_index;
+    a.num_cb = h->num_cb;
+    a.logits_out = h->logits_out;
+    a.finished = h->finished;
+    a.row_slot = h->row_slot;
+    a.noise_u = h->noise_u;
+    a.noise_draws = h->noise_draws;
+    a.noise_ld = h->noise_ld;
+    FSB_TRY(launch_sample(a, st));
+    FSB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
+int fsb_op_frame_end(const int32_t* d_cur_tok, int32_t* d_out_tokens, int32_t* d_n_out, int32_t* d_pos,
+                     const int32_t* d_row_slot, const int32_t* d_set_pos_rows, const int32_t* d_row_pos_src,
+                     unsigned long long* d_step, int rows, int ncols, int T_cap, const fsb_op_slot_ctl* ctl,
+                     void* stream) {
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    FSB_CHECK(rows >= 1 && ncols >= 1 && ncols <= 32 && T_cap >= 1 && d_step, "frame_end hook: shape");
+    FSB_CHECK(!d_set_pos_rows || d_row_pos_src, "frame_end hook: set_pos_rows needs row_pos_src");
+    FrameEndArgs a{};
+    FSB_TRY(hook_slot_ctl(ctl, &a.ctl));
+    FSB_CHECK(!a.ctl.state || a.ctl.limit, "frame_end hook: slot control needs state and limit");
+    a.cur_tok = d_cur_tok;
+    a.out_tokens = d_out_tokens;
+    a.n_out = d_n_out;
+    a.pos = d_pos;
+    a.row_slot = d_row_slot;
+    a.set_pos_rows = d_set_pos_rows;
+    a.row_pos_src = d_row_pos_src;
+    a.step = d_step;
+    a.rows = rows; a.ncols = ncols; a.T_cap = T_cap;
+    FSB_TRY(launch_frame_end(a, st));
+    FSB_CUDA(cudaStreamSynchronize(st));
+    return 0;
+}
+
 }  // extern "C"

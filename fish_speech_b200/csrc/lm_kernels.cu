@@ -730,7 +730,8 @@ __global__ void __launch_bounds__(kSampleThreads) sample_kernel(SampleArgs a) {
         if (w < (two ? 2 : 1)) {
             const float T = w == 0 ? temperature : 1.0f;
             const float tp = w == 0 ? top_p : 0.9f;
-            const float Tc = fmaxf(T, 1e-5f);
+            // torch.clip(temperature, min=1e-5) on the bf16 temperature tensor clamps to bf16(1e-5)
+            const float Tc = fmaxf(T, 1.0013580322265625e-05f);
             // survivors: rank 0 always; rank r kept iff cum[r] <= top_p (and r < top_k, implied)
             int ns = 1;
             while (ns < nsel && !(sel_cum[ns] > tp)) ++ns;

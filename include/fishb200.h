@@ -278,6 +278,54 @@ int fsb_op_attn_decode(const float* d_ws, const int32_t* d_nparts, int tiles, in
                        const int32_t* d_row_seq, const int32_t* d_row_pos, void* d_out, int rows, int H, int Hkv,
                        int Dh, int S, int lcap, int bf16_math, int kv_only, float eps, void* stream);
 
+/* Per-slot request control of the frame kernels (SlotCtl, csrc/lm_kernels.cuh): with `state` set, the sampler takes
+ * temperature / top_p / top_k / seed and its RNG counter (n_out) from these [slots] arrays, and idle (0) and
+ * finished (2) slots are left untouched. All NULL = no slot control. */
+typedef struct {
+    int32_t* state;
+    const int32_t* limit;
+    const float* temperature;
+    const float* top_p;
+    const int32_t* top_k;
+    const unsigned long long* seed;
+    const int32_t* n_out;
+} fsb_op_slot_ctl;
+/* Every field of the sampler's SampleArgs; the logits are the slot-ordered sums of the partial set (ws, nparts,
+ * tiles = ceil(n / 128), max_parts) rounded to bf16. Rows index the partial set, `row_slot` (optional) maps a row to
+ * the slot whose state it reads and writes. */
+typedef struct {
+    const float* ws;
+    const int32_t* nparts;
+    int tiles, max_parts;
+    int n, rows;
+    float temperature, top_p;
+    int top_k;
+    int slow, n_sem, sem_begin, im_end_id, codebook_size;
+    int use_ras;
+    int32_t* ras_window; /* [slots][10] */
+    int ras_update;
+    unsigned long long seed;
+    const unsigned long long* rng_offset; /* device counter, may be NULL (0) */
+    int draw_id;
+    int32_t* cur_tok; /* [slots][num_cb + 1] */
+    int cb_index, num_cb;
+    float* logits_out;     /* optional [slots][n] */
+    int32_t* finished;     /* optional [slots] */
+    const int32_t* row_slot;
+    const float* noise_u;  /* optional uniforms of slot 0, see fsb_lm_set_sampler_noise */
+    int noise_draws, noise_ld;
+    fsb_op_slot_ctl ctl;
+} fsb_op_sample_args;
+/* sample_kernel (top-k / top-p / temperature / RAS / Philox draw) through launch_sample. */
+int fsb_op_sample(const fsb_op_sample_args* a, void* stream);
+/* frame_end_kernel + the step counter increment through launch_frame_end: out_tokens [slots][ncols][T_cap] gets
+ * cur_tok [slots][ncols] at n_out[slot], n_out and pos advance (pos = row_pos_src[set_pos_rows[row]] + 1 when
+ * set_pos_rows is given), and *d_step += 1. ctl (may be NULL) needs state and limit only. */
+int fsb_op_frame_end(const int32_t* d_cur_tok, int32_t* d_out_tokens, int32_t* d_n_out, int32_t* d_pos,
+                     const int32_t* d_row_slot, const int32_t* d_set_pos_rows, const int32_t* d_row_pos_src,
+                     unsigned long long* d_step, int rows, int ncols, int T_cap, const fsb_op_slot_ctl* ctl,
+                     void* stream);
+
 /* The decode attention (fsb_op_attn_decode, the decode frame) keeps one fp32 score per position and head in shared
  * memory; contexts longer than the buffer are walked in chunks, bit-identically (csrc/lm_kernels.cu attend()).
  * positions > 0 forces a smaller chunk; 0 = automatic. */
